@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config C]          # product arm (one process per GPU under torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K ... [--config C]  # reference arm: the CPU oracle of the same path, rank 0 only
+  python bench.py ... --dump-outputs DIR                                # product arm, plus the last timed step's outputs as DIR/*.npy
 
 Workloads (BASELINE.json `configs`, SURVEY.md §8d; per-GPU shards of the image-sharded global batches):
   --config 1 (default, the configuration the metric is quoted on)  ViT-H, 8 x 1024x1024, 80-class COCO vocabulary (Lt = 512), detection
@@ -221,6 +222,46 @@ def ncu_traffic(kernel_tag):
     return None, None
 
 
+DUMP_CAP = 1 << 18          # elements kept per array; a larger array is dumped as a fixed, seeded sample of this many elements
+DUMP_BUDGET = 64 << 20      # bytes of all dumped arrays together
+
+
+def dump_outputs(out, path):
+    """Writes every tensor of the hot path's result (nested dicts / lists flattened to dotted names, e.g. aux.hs.5) as
+    <path>/<name>.npy: floating point and bool as float32, integers (top-k indices) as float64.  An array of more than DUMP_CAP
+    elements is replaced by its elements at DUMP_CAP flat positions drawn with seed 0 and sorted, the same positions in every run,
+    so that the dumps of two builds compare element for element."""
+    import numpy as np
+    import torch
+    tensors = {}
+
+    def walk(name, v):
+        if torch.is_tensor(v):
+            tensors[name] = v
+        elif isinstance(v, dict):
+            for k, x in v.items():
+                walk(f"{name}.{k}" if name else str(k), x)
+        elif isinstance(v, (list, tuple)):
+            for i, x in enumerate(v):
+                walk(f"{name}.{i}", x)
+    walk("", out)
+    arrays = {}
+    for name, t in sorted(tensors.items()):
+        t = t.detach()
+        if t.numel() > DUMP_CAP:
+            idx = torch.randint(t.numel(), (DUMP_CAP,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        exact_ints = not t.is_floating_point() and t.dtype != torch.bool
+        arrays[name] = (t.double() if exact_ints else t.float()).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BUDGET:
+        raise RuntimeError(f"--dump-outputs: {len(arrays)} arrays take {total} bytes, more than {DUMP_BUDGET}")
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    print(f"[bench] dumped {len(arrays)} arrays ({total / 2**20:.1f} MiB) of the last timed step to {path}", file=sys.stderr)
+
+
 def run_product(args, cfg):
     import torch
     import torch.distributed as dist
@@ -306,10 +347,12 @@ def run_product(args, cfg):
             s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             s.record()
             for _ in range(args.steps):
-                hot_step()
+                out = hot_step()
             e.record()
             barrier()
         ms = s.elapsed_time(e)
+        if args.dump_outputs and rank == 0:      # before the steps below can reuse any buffer of the last timed step
+            dump_outputs(out, args.dump_outputs)
         launches = _lib.launch_count() - launches0
         if graphed is not None:          # replayed launches are not re-counted by the library: kernels per capture x replays
             launches = graphed.launches_per_replay * args.steps
@@ -457,7 +500,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch the hot step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--ref-budget-s", type=float, default=240.0, help="wall-clock budget of the --impl reference run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (product arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     # stdout carries exactly one JSON line.  NCCL_DEBUG is left as the caller set it (the driver reads the NCCL log for its
     # evidence); NCCL prints its log to stdout by default, so it is routed to stderr instead of being silenced.
     if int(os.environ.get("WORLD_SIZE", "1")) > 1 and os.environ.get("NCCL_DEBUG", ""):

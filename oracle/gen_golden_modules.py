@@ -22,6 +22,10 @@ same outputs, which pins these rows of SURVEY.md §8a to the reference itself:
   ref_maskclip.pt     a22/f2  open_vocab/clip.py MaskCLIP (mask tokens, per-query attention masks, logit ensembling) and ClipAdapter._encode_text
                               on top of the restated open_clip 2.0.2 model (absent third-party dependency: hipie_oracle/clip.py), and
                               hipie_img.py HIPIE_IMG.get_clip_logits (MUL and ADD fusion, seen / unseen weights)
+  ref_configs.json            projects/HIPIE/configs: the r50 / ViT-H training and ADE eval YAMLs with their _BASE_ and MaskDINO
+                              config chains (the config surface, hipie_b200/config.py, has to load them unchanged)
+  ref_msda_binding.pt a12     ops/functions/ms_deform_attn_func.py: MSDeformAttnFunction's call of the pybind op (argument order)
+                              and ms_deform_attn_core_pytorch on the same inputs
 """
 import copy
 import os
@@ -390,8 +394,65 @@ def gen_maskclip():
     print("ref_maskclip.pt", tuple(out["mask_embed"].shape), tuple(out["mask_pred_open_logits"].shape), {k: tuple(v.shape) for k, v in fused.items()})
 
 
+CONFIGS = ["training/r50.yaml", "training/vit_huge_32g.yaml", "eval/image_joint_vit_huge_32g_pan_maskdino_ade_test.yaml"]
+
+
+def gen_configs():
+    """projects/HIPIE/configs: the YAMLs the config tests load, with every file their _BASE_ chains and MASKDINO.CONFIG_PATH
+    reach, as parsed by yaml.safe_load and keyed by the path under the reference root, so that a test can lay the same tree out
+    again and load it through hipie_b200.config."""
+    import json
+    import yaml
+    cfg_root = "projects/HIPIE/configs"
+    tree, todo = {}, [f"{cfg_root}/{c}" for c in CONFIGS]
+    while todo:
+        rel = os.path.normpath(todo.pop())
+        if rel in tree:
+            continue
+        with open(os.path.join(ref_import.REF_ROOT, rel)) as f:
+            d = tree[rel] = yaml.safe_load(f)
+        if "_BASE_" in d:
+            todo.append(os.path.join(os.path.dirname(rel), d["_BASE_"]))
+        path = d.get("MODEL", {}).get("MASKDINO", {}).get("CONFIG_PATH")
+        if path:
+            todo.append(path)
+    for d in tree.values():
+        assert yaml.safe_load(yaml.safe_dump(d)) == d          # the test writes them back out with safe_dump
+    with open(os.path.join(OUT, "ref_configs.json"), "w") as f:
+        json.dump({"configs": CONFIGS, "root": cfg_root, "files": dict(sorted(tree.items()))}, f, indent=1)
+        f.write("\n")
+    print("ref_configs.json", sorted(tree))
+
+
+def gen_msda_binding():
+    """ops/functions/ms_deform_attn_func.py: the positional argument list MSDeformAttnFunction.forward passes to the pybind op
+    `MultiScaleDeformableAttention.ms_deform_attn_forward` (recorded by a stand-in module), and ms_deform_attn_core_pytorch on the
+    same seeded inputs."""
+    seen = []
+    msda = types.ModuleType("MultiScaleDeformableAttention")
+    msda.ms_deform_attn_forward = lambda *args: seen.append(args) or torch.zeros(())
+    prev, sys.modules["MultiScaleDeformableAttention"] = sys.modules.get("MultiScaleDeformableAttention"), msda
+    f = ref_import._load_file("ref_ms_deform_attn_func", f"{ref_import.HIPIE}/models/deformable_detr/ops/functions/ms_deform_attn_func.py")
+    sys.modules["MultiScaleDeformableAttention"] = prev
+    g = torch.Generator().manual_seed(41)
+    inputs = dict(value=torch.rand(1, 20, 2, 4, generator=g), shapes=torch.tensor([(4, 4), (2, 2)], dtype=torch.long),
+                  level_start_index=torch.tensor([0, 16]), sampling_loc=torch.rand(1, 3, 2, 2, 2, 2, generator=g),
+                  attn_weight=torch.rand(1, 3, 2, 2, 2, generator=g))
+    im2col_step = 64
+    with torch.no_grad():
+        f.MSDeformAttnFunction.apply(*inputs.values(), im2col_step)
+        core = f.ms_deform_attn_core_pytorch(inputs["value"], inputs["shapes"], inputs["sampling_loc"], inputs["attn_weight"])
+    (args,) = seen
+    call = [next(n for n, t in inputs.items() if a is t) if torch.is_tensor(a) else ("im2col_step" if a == im2col_step else None)
+            for a in args]
+    assert None not in call
+    torch.save(dict(inputs=inputs, im2col_step=im2col_step, call=call, core=core), os.path.join(OUT, "ref_msda_binding.pt"))
+    print("ref_msda_binding.pt", call, tuple(core.shape))
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
-    which = sys.argv[1:] or ["vit", "transformer", "maskdino", "condinst", "bert", "postproc", "prompts", "r50", "maskclip"]
+    which = sys.argv[1:] or ["vit", "transformer", "maskdino", "condinst", "bert", "postproc", "prompts", "r50", "maskclip", "configs",
+                             "msda_binding"]
     for w in which:
         globals()["gen_" + w]()

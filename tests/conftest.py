@@ -21,6 +21,22 @@ def golden_dir():
 
 
 @pytest.fixture(scope="session")
+def ref_configs(tmp_path_factory):
+    """The reference's config YAMLs (tests/golden/ref_configs.json) written out in their original layout, so that _BASE_ and
+    MASKDINO.CONFIG_PATH resolve as they do in the reference tree.  Returns the configs directory."""
+    import json
+    import yaml
+    with open(os.path.join(GOLDEN, "ref_configs.json")) as f:
+        g = json.load(f)
+    root = tmp_path_factory.mktemp("reference")
+    for rel, d in g["files"].items():
+        p = root / rel
+        p.parent.mkdir(parents=True, exist_ok=True)
+        p.write_text(yaml.safe_dump(d))
+    return root / g["root"]
+
+
+@pytest.fixture(scope="session")
 def cuda():
     import torch
     if not torch.cuda.is_available():

@@ -1,18 +1,16 @@
-"""CPU: the reference's own YAMLs load unchanged through the config surface (skipped where /root/reference is absent)."""
+"""CPU: the reference's own YAMLs (tests/golden/ref_configs.json, laid out by the `ref_configs` fixture) load unchanged through
+the config surface."""
 import os
 
 import pytest
 
-REF = "/root/reference/projects/HIPIE/configs"
 
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference configs only exist in the build container")
 @pytest.mark.parametrize("rel", ["training/r50.yaml", "training/vit_huge_32g.yaml",
                                  "eval/image_joint_vit_huge_32g_pan_maskdino_ade_test.yaml"])
-def test_reference_yaml_loads(rel):
+def test_reference_yaml_loads(rel, ref_configs):
     from hipie_b200.config import setup_cfg
     from hipie_b200.modeling.hipie_img import hp_from_cfg
-    cfg = setup_cfg(os.path.join(REF, rel), ["MODEL.DEVICE", "cuda"])
+    cfg = setup_cfg(os.path.join(ref_configs, rel), ["MODEL.DEVICE", "cuda"])
     assert cfg.MODEL.META_ARCHITECTURE == "HIPIE_IMG"
     assert cfg.MODEL.DDETRS.TWO_STAGE_NUM_PROPOSALS == 900 and cfg.MODEL.DDETRS.TWO_STAGE_NUM_BG_PROPOSALS == 10
     assert cfg.MODEL.MASKDINO.ENABLED is True
